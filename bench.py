@@ -26,7 +26,10 @@ Workloads (BASELINE.json `configs`):
 oracle/build_ref.sh) through its own public API on the same workload and protocol -- the reference is a GPU library, so
 its arm runs on the GPU; when the library is missing the arm falls back to the CPU oracle port.
 
-Launch: python bench.py [--gpus N --steps K --warmup W]; for N>1 under torch.distributed.run.
+Launch: python bench.py [--gpus N --steps K --warmup W] [--dump-outputs DIR]; for N>1 under torch.distributed.run.
+Every workload, the headline and each of the configs, times K steps.  --dump-outputs writes what the last timed step of the
+headline returned (chi2 / lambda / trials / pcg_iters per iteration, q, t, Xw) as DIR/<name>.npy; the inputs are the fixture or
+a seeded graph, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import dataclasses
@@ -173,8 +176,9 @@ class Runner:
             eng.set_comm(self.rank, self.world, self.uid_fn())
         return eng
 
-    def measure(self, prob, rk, steps, warmup, protocol_warmup=False, stages=True, clocks=None):
-        """returns a dict with value / e2e / roofline / stage times for one workload"""
+    def measure(self, prob, rk, steps, warmup, protocol_warmup=False, stages=True, clocks=None, keep_outputs=False):
+        """returns a dict with value / e2e / roofline / stage times for one workload; with keep_outputs, also "outputs": what the
+        last timed optimize(10) returned to its caller (per-iteration statistics and the final q / t / Xw)"""
         torch = self.torch
         pkg = self.pkg
         E = prob.nedges
@@ -243,6 +247,11 @@ class Runner:
                 dev_ms.append(self.max_over_ranks(a.elapsed_time(b))); iters_done = len(stats)
                 pcg_total = sum(s["pcg_iters"] for s in stats)
         launches = eng.launch_count() - launches0
+        outputs = None
+        if keep_outputs:
+            q, t, Xw = eng.state()
+            outputs = {"chi2": [s["chi2"] for s in stats], "lambda": [s["lambda_"] for s in stats], "trials": [s["trials"] for s in stats],
+                       "pcg_iters": [s["pcg_iters"] for s in stats], "q": q, "t": t, "Xw": Xw}
         pcg_ms = (1e3 * eng.time_profile()["6: Numerical Decomposition"] - pcg_ms0) / max(steps, 1)
         if clocks is not None:
             clocks.stop_flag.set(); clocks.join(timeout=3)
@@ -256,7 +265,7 @@ class Runner:
                        "window": "set_problem(H2D from pinned host buffers + full structure build, structure reuse switched OFF) + optimize(10) + get_state(D2H) == reference's initialize()+optimize(10)"},
                "e2e_reuse": {"value": E * e2e_iters / (float(np.mean(reuse_ms)) * 1e-3), "unit": "edge-iterations/s", "ms_per_step": float(np.mean(reuse_ms)), "structure_reuses": reuses,
                              "window": "the same window with the engine's default structure reuse: the topology is unchanged between calls, so set_problem only uploads values (SURVEY 8 f-2)"},
-               "profile_ms_e2e_step": {k: round(1e3 * v, 4) for k, v in prof.items()}, "prob": prob}
+               "profile_ms_e2e_step": {k: round(1e3 * v, 4) for k, v in prof.items()}, "prob": prob, "outputs": outputs}
         # ---------------- roofline of the J+H landmark-pass kernel + per-stage device times (L2 flushed between reps)
         if stages:
             eng.reset_state(); eng.linearize()
@@ -287,6 +296,27 @@ def cpu_reference_chi2(prob, rk):
     o = oracle.Oracle(prob, rk[0], rk[1])
     t0 = time.perf_counter(); chi, lam_o, tr = o.optimize(LM_ITERS); dt = time.perf_counter() - t0
     return chi, prob.nedges * len(chi) / dt, dt
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(outputs, out_dir):
+    """--dump-outputs: one <name>.npy per output of the last timed step, float32 / float64, so that two builds can be compared
+    output for output.  Beyond 64 MB in all, Xw keeps a fixed seeded sample of its rows, whose indices go to Xw_rows.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {}
+    for name, v in outputs.items():
+        a = np.asarray(v)
+        arrays[name] = a if a.dtype in (np.float32, np.float64) else a.astype(np.float64)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        Xw = arrays["Xw"]
+        k = (DUMP_BYTES - (total - Xw.nbytes)) // (Xw.itemsize * Xw.shape[1] + 8)
+        rows = np.sort(np.random.default_rng(0).choice(len(Xw), k, replace=False))
+        arrays["Xw"], arrays["Xw_rows"] = Xw[rows], rows.astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def run_e2e_cpp(pkg, workload, graph, robust, steps, warmup, reuse=True):
@@ -399,7 +429,11 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the C1..C5 array (and, on several GPUs, the secondary workload)")
     ap.add_argument("--no-cpp", action="store_true")
     ap.add_argument("--child", action="store_true", help=argparse.SUPPRESS)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (chi2, lambda, trials, pcg_iters per iteration; q, t, Xw) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps this engine's outputs: use it with --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -449,7 +483,9 @@ def main():
     graph = load_graph(pkg, args.workload)
     prob0 = pkg.graphio.flatten(graph)
     clocks = ClockSampler(local)
-    m = run.measure(prob0, rk, args.steps, args.warmup, protocol_warmup=args.protocol_warmup, clocks=clocks)
+    m = run.measure(prob0, rk, args.steps, args.warmup, protocol_warmup=args.protocol_warmup, clocks=clocks, keep_outputs=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(m["outputs"], args.dump_outputs)
     E, sizes = m["E"], m["sizes"]
     tpath = os.path.join(ROOT, "profiles", "jh_traffic.json")
     if os.path.exists(tpath) and world == 1:
@@ -508,15 +544,16 @@ def main():
     if not args.no_configs and not explicit and not args.fp32:
         if world == 1:
             configs = [config_entry("C2", args.workload, args.robust, False, m, chi_oracle, oracle_kind)]
-            plan = [("C1", "ba_kitti_07", "none", False, 3, 3), ("C1", "ba_kitti_07", "huber", False, 3, 3), ("C2", "ba_kitti_00", "huber", False, 3, 3),
-                    ("C5", "ba_kitti_00", "none", True, 3, 3), ("C5-mixed", "ba_kitti_00", "none", "mixed", 3, 3),
-                    ("C3", "synth_mono_5m", "huber", False, 2, 1), ("C4", "synth_stereo_10m", "huber", False, 2, 1)]
-            for name, wl, rb, f32, st, wu in plan:
+            # (config, workload, robust kernel, precision, warm-up steps); every config times --steps steps
+            plan = [("C1", "ba_kitti_07", "none", False, 3), ("C1", "ba_kitti_07", "huber", False, 3), ("C2", "ba_kitti_00", "huber", False, 3),
+                    ("C5", "ba_kitti_00", "none", True, 3), ("C5-mixed", "ba_kitti_00", "none", "mixed", 3),
+                    ("C3", "synth_mono_5m", "huber", False, 1), ("C4", "synth_stereo_10m", "huber", False, 1)]
+            for name, wl, rb, f32, wu in plan:
                 wl, _ = resolve_workload(wl)
                 try:
                     p = build_problem(pkg, wl)
                     r2 = Runner(pkg, local, rank, world, fp32=(f32 is True), mixed=(f32 == "mixed"))
-                    mm = r2.measure(p, KERNELS[rb], st, wu, protocol_warmup=wl.startswith("ba_"))
+                    mm = r2.measure(p, KERNELS[rb], args.steps, wu, protocol_warmup=wl.startswith("ba_"))
                     oc, ok_ = None, None
                     if not f32:
                         if wl.startswith("ba_"):
@@ -531,7 +568,7 @@ def main():
                     if f32:
                         # C5: chi2 tolerance vs fp64 = deviation of the fp32 trajectory from the fp64 run of the same protocol
                         ent["chi2_rel_diff_vs_fp64"] = float(np.abs(np.array(mm["chi2"]) - np.array(m["chi2"])).max() / np.abs(m["chi2"]).max()) if len(mm["chi2"]) == len(m["chi2"]) else None
-                    ent["steps"], ent["warmup"] = st, wu
+                    ent["steps"], ent["warmup"] = args.steps, wu
                     configs.append(ent)
                     del mm, p
                 except Exception as ex:
@@ -545,7 +582,7 @@ def main():
         else:
             try:
                 p = build_problem(pkg, "kitti00_shaped")
-                mm = run.measure(p, KERNELS["none"], 3, 3, stages=False)
+                mm = run.measure(p, KERNELS["none"], args.steps, 3, stages=False)
                 oc = gl.get("kitti00_shaped_none", {}).get("chi2")
                 line["secondary"] = config_entry("kitti00_shaped (strong scaling of a latency-bound graph)", "kitti00_shaped", "none", False, mm, oc, "golden (tests/golden/oracle_large.json)" if oc else None)
             except Exception as ex:

@@ -45,6 +45,14 @@ def have_fixture(name):
     return os.path.exists(fixture_path(name))
 
 
+SUBGRAPHS = ("kitti07_sub", "kitti00_sub")   # stored pieces of the two real graphs (tests/golden/make_subgraphs.py)
+
+
+def load_subgraph(name):
+    with np.load(os.path.join(ROOT, "tests", "golden", name + ".npz")) as z:
+        return {k: z[k].astype(np.int32 if z[k].dtype.kind == "i" else np.float64) for k in z.files}
+
+
 @pytest.fixture(scope="session")
 def problems(pkg):
     """cache of flattened problems by name"""
@@ -54,6 +62,8 @@ def problems(pkg):
         if name not in cache:
             if name.startswith("ba_"):
                 g = pkg.graphio.read_graph(fixture_path(name))
+            elif name in SUBGRAPHS:
+                g = load_subgraph(name)
             else:
                 g = pkg.synth.make_config(name)
             cache[name] = pkg.graphio.flatten(g)
