@@ -182,14 +182,13 @@ def pcg5_plan_host(prob, world=1, num_sms=148, max_aggregates=74):
 class Engine:
     """One optimizer instance on one GPU (reference: one CudaBundleAdjustment per thread/device)."""
 
-    def __init__(self, device=-1, use_fp32=False, pcg_max_iters=0, pcg_tol=0.0, pcg_variant=0, structure_on_host=False, jh_variant=0, schur_variant=0,
+    def __init__(self, device=-1, use_fp32=False, pcg_max_iters=0, pcg_tol=0.0, pcg_variant=0, structure_on_host=False, jh_variant=0,
                  coarse_refresh=0, two_level_switch=0, max_aggregates=0):
         self.L = load_library()
         res = (C.c_int * 7)()
         res[0] = int(pcg_variant)
         res[1] = int(bool(structure_on_host))
         res[2] = int(jh_variant)
-        res[3] = int(schur_variant)
         res[4] = int(coarse_refresh)
         res[5] = int(two_level_switch)
         res[6] = int(max_aggregates)

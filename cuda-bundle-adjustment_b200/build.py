@@ -6,7 +6,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libcuba_b200.so")
 SOURCES = ["cuba_engine.cu", "cuba_structure.cpp", "cuba_api.cpp"]
-HEADERS = ["cuba_kernels.cuh", "cuba_jh4.cuh", "cuba_schur3.cuh", "cuba_schur5.cuh", "cuba_pcg2.cuh", "cuba_pcg3.cuh", "cuba_pcg4.cuh", "cuba_pcg5.cuh", "cuba_pcg5t.cuh", "cuba_coarse_dense.cuh", "cuba_peer_reduce.cuh", "cuba_schur2.cuh", "cuba_structure_gpu.cuh", "cuba_math.cuh", "cuba_structure.h",
+HEADERS = ["cuba_kernels.cuh", "cuba_jh4.cuh", "cuba_schur3.cuh", "cuba_pcg2.cuh", "cuba_pcg3.cuh", "cuba_pcg4.cuh", "cuba_pcg5.cuh", "cuba_pcg5t.cuh", "cuba_coarse_dense.cuh", "cuba_peer_reduce.cuh", "cuba_structure_gpu.cuh", "cuba_math.cuh", "cuba_structure.h",
            "../../include/cuba_b200.h", "../../include/cuda_bundle_adjustment.h", "../../include/cuda_bundle_adjustment_types.h"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = (["-DCUBA_JH4_DEBUG"] if os.environ.get("CUBA_JH4_DEBUG") else []) + ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",

@@ -23,10 +23,8 @@
 #include "cuba_pcg5t.cuh"
 #include "cuba_coarse_dense.cuh"
 #include "cuba_peer_reduce.cuh"
-#include "cuba_schur2.cuh"
 #include "cuba_jh4.cuh"
 #include "cuba_schur3.cuh"
-#include "cuba_schur5.cuh"
 #include "cuba_structure.h"
 #include "cuba_structure_gpu.cuh"
 
@@ -203,14 +201,10 @@ struct Engine : EngineBase {
 	cudaStream_t stream = nullptr;
 	int numSMs = 0;
 	int ntiles = 0, nPoseBlocks = 0, nChiBlocks = 0;
-	int tileSize = TILE;    // 256 or 128, from cfg.reserved[2]
-	int jhMinBlocks = 2;
-	bool jhV2 = true;       // k_linearize_landmark2 (pose window in smem + TMA bulk store of Hpl)
-	bool jhV3 = true;       // k_linearize_landmark3 (v2 + persistent CTAs with a cp.async double-buffered input stage)
-	int jh3Grid = 0, nChiLin = 0;
-	// warp-tile J+H landmark pass (cuba_jh4.cuh)
+	int nChiLin = 0;
+	// warp-tile J+H landmark pass (cuba_jh4.cuh); otherwise the tile kernel k_linearize_landmark
 	bool jhV4 = true;
-	int ntW = 0, jh4Grid = 0, jh4HasBig = 0, jh4MinB = 4, jh4Nst = 2;
+	int ntW = 0, jh4Grid = 0, jh4HasBig = 0;
 	const void* jh4AttrSet = nullptr;
 	int* jh4Host = nullptr;      // pinned: {number of warp tiles, any cut landmark}
 	bool jh4Pending = false;
@@ -218,21 +212,6 @@ struct Engine : EngineBase {
 	DBuf<jh4::WTile> w_tile;
 	DBuf<jh4::Rec> w_rec;
 	DBuf<double> w_bigPartial;
-	DBuf<TileInfo> tileInfo;
-	// tile-local Schur (cuba_schur2.cuh)
-	bool useSchur2 = true;
-	bool useSchur5 = false;  // landmark tiles + DMMA (cuba_schur5.cuh), fp64 only
-	int s5Ntiles = 0;
-	DBuf<int> s5TileLm;
-	DBuf<TileInfo> s5TileInfo;
-	DBuf<int4> s5SegRec;
-	DBuf<unsigned int> s5Off;
-	int s2Nseg = 0, s2Nvalid = 0;
-	DBuf<unsigned long long> s2_key, s2_keyS, s2_key3, s2_key3S;
-	DBuf<int> s2_val, s2_valS, s2_head, s2_segId, s2_segStart, s2_segTile, s2_segDest, s2_val3, s2_val3S, s2_segRank, s2_rankDest, s2_tileSegPtr, s2_destSegPtr, s2_p2i, s2_p2j;
-	DBuf<schur2::Counts> s2_counts;
-	DBuf<T> s2_partial;
-	DBuf<int> tilePose0, tilePoseN;
 	int cur = 0;            // current state buffer
 	bool trialValid = false;
 	// state
@@ -248,11 +227,6 @@ struct Engine : EngineBase {
 	bool mixed = false;
 	bool upperReduce = false;   // k_schur3 writes the upper blocks into uVal; one all-reduce of uVal | bsc, then k_expand_upper
 	DBuf<int> prodPtr, prodI, prodJ, prodL, blkRow, blkCol, u2f, u2fT, fRowPtr, fColInd;
-	bool useSchur3 = true;
-	// pcg
-	DBuf<T> pr, pz, pq, pp0, pp1, Minv;
-	DBuf<double> pcgPartial;
-	int pcgGrid = 0;
 	// pcg v2 (cuba_pcg2.cuh)
 	DBuf<T> fHat, Linv, vR0, vR1, vS0, vS1, vW0, vW1, vP, vY;
 	DBuf<int> fLocal, ctaRow, needPtr, needCol;
@@ -409,23 +383,8 @@ struct Engine : EngineBase {
 		reusable = false;
 		hostStructureValid = false;
 		shardBoundValid = false;
-		// landmark-tile variant: 0/1 = 256 edges, 2 CTAs/SM; 2 = 256, 3 CTAs/SM; 3 = 128, 4 CTAs/SM; 4 = 128, 6 CTAs/SM
-		switch (cfg.reserved[2]) {
-		case 2: tileSize = 256; jhMinBlocks = 3; break;
-		case 3: tileSize = 128; jhMinBlocks = 4; break;
-		case 4: tileSize = 128; jhMinBlocks = 6; break;
-		case 1: tileSize = 256; jhMinBlocks = 2; break;
-		default: tileSize = JH2_TL; jhMinBlocks = 4; break;
-		}
-		// k_linearize_landmark4: 0 = two-stage pipeline, 4 CTAs of 4 warps per SM (default); 8/9 = 5/6 CTAs per SM; 7 = three stages
-		jhV4 = (cfg.reserved[2] == 0 || (cfg.reserved[2] >= 7 && cfg.reserved[2] <= 9)) && sizeof(T) == 8;
-		jh4Nst = cfg.reserved[2] == 7 ? 3 : 2;
-		jh4MinB = cfg.reserved[2] == 8 ? 5 : (cfg.reserved[2] == 9 ? 6 : 4);
-		jhV3 = cfg.reserved[2] == 6 && sizeof(T) == 8;
-		jhV2 = cfg.reserved[2] == 5 && sizeof(T) == 8;
-		if (cfg.reserved[2] == 5) { tileSize = JH2_TL; jhMinBlocks = 4; }
-		// (the bulk copy needs 16-byte multiples: 144-byte fp64 blocks qualify, 72-byte fp32 blocks do not)
-		if (cfg.reserved[2] == 0 && sizeof(T) != 8) { tileSize = 128; jhMinBlocks = 6; }
+		// J+H landmark pass: k_linearize_landmark4 in fp64; k_linearize_landmark in fp32 and, for the agreement test, with cfg.reserved[2] == 4
+		jhV4 = cfg.reserved[2] == 0 && sizeof(T) == 8;
 		int rc = (cfg.reserved[1] == 1) ? build_on_host(p) : build_on_gpu(p);
 		if (rc) return rc;
 		tmark("structure built");
@@ -494,7 +453,7 @@ struct Engine : EngineBase {
 	int build_on_host(const cuba_problem* p)
 	{
 		const char* err = "";
-		if (!build_structure(p->Pall, p->numP, p->Lall, p->numL, p->E2, p->idx2, p->E3, p->idx3, rank, world, tileSize, S, &err))
+		if (!build_structure(p->Pall, p->numP, p->Lall, p->numL, p->E2, p->idx2, p->E3, p->idx3, rank, world, LM_TILE, S, &err))
 			return fail(CUBA_ERR_INVALID, err);
 		hostStructureValid = true;
 		const int eL = S.eLocal;
@@ -623,11 +582,9 @@ struct Engine : EngineBase {
 		CUDA_TRY(tilePtr.alloc((size_t)numL + 2));
 		KLAUNCH(k_tile_ptr, numL + 2, lmPtr.p, numL, eL, tilePtr.p);
 		const int tb = std::min(S.lmBeg, numL), te = std::min(S.lmEnd, numL) + (S.lmEnd > numL ? 1 : 0);
-		// windows a little shorter than the CTA so that the tail of a tile's last landmark usually still fits one chunk
-		const int window = tileSize == 128 ? JH3_WINDOW : tileSize - 16;
-		const int nt = (eL + window - 1) / window;
+		const int nt = (eL + LM_WINDOW - 1) / LM_WINDOW;
 		CUDA_TRY(tileLm.alloc((size_t)nt + 1));
-		KLAUNCH(k_tiles, nt + 1, tilePtr.p, tb, te, window, nt, tileLm.p);
+		KLAUNCH(k_tiles, nt + 1, tilePtr.p, tb, te, LM_WINDOW, nt, tileLm.p);
 		ntiles = nt;
 		// 4. pose-major stream (free poses only)
 		CUDA_TRY(g_k32.alloc(eL)); CUDA_TRY(g_k32S.alloc(eL)); CUDA_TRY(g_pval.alloc(eL)); CUDA_TRY(g_psrc.alloc(eL));
@@ -740,7 +697,7 @@ struct Engine : EngineBase {
 		else CUDA_TRY(Hpl.alloc(18 * (size_t)S.nhplLocal));
 		CUDA_TRY(invHll.alloc(9 * nL));
 		CUDA_TRY(fVal.alloc(36 * (size_t)S.nfull + 6 * nP)); bsc.alias(fVal.p + 36 * (size_t)S.nfull, 6 * nP);
-		upperReduce = world > 1 && (cfg.reserved[3] == 0 || cfg.reserved[3] == 3 || cfg.use_fp32 == 2) && S.numP > 0 && S.numL > 0;
+		upperReduce = world > 1 && S.numP > 0 && S.numL > 0;
 		if (upperReduce) {
 			uCount = 36 * (size_t)S.nblk + 6 * nP;
 			const size_t need = ((uCount + 1) & ~(size_t)1) + 64;          // + the signal block of the peer all-reduce
@@ -765,8 +722,6 @@ struct Engine : EngineBase {
 			}
 		}
 		CUDA_TRY(xp.alloc(6 * nP)); CUDA_TRY(xl.alloc(3 * nL));
-		CUDA_TRY(pr.alloc(6 * nP)); CUDA_TRY(pz.alloc(6 * nP)); CUDA_TRY(pq.alloc(6 * nP)); CUDA_TRY(pp0.alloc(6 * nP)); CUDA_TRY(pp1.alloc(6 * nP));
-		CUDA_TRY(Minv.alloc(36 * nP));
 		// landmarks outside this rank's shard keep zero Hll/bl/xl (they are never touched locally)
 		if (nL) CUDA_TRY(cudaMemsetAsync(Hll.p, 0, sizeof(T) * 9 * nL, stream));
 		if (nL) CUDA_TRY(cudaMemsetAsync(bl.p, 0, sizeof(T) * 3 * nL, stream));
@@ -774,52 +729,11 @@ struct Engine : EngineBase {
 		if (nP) CUDA_TRY(cudaMemsetAsync(xp.p, 0, sizeof(T) * 6 * nP, stream));
 		if (nP) CUDA_TRY(cudaMemsetAsync(Hpp.p, 0, sizeof(T) * 36 * nP, stream));
 		if (nP) CUDA_TRY(cudaMemsetAsync(bp.p, 0, sizeof(T) * 6 * nP, stream));
-		CUDA_TRY(tilePose0.alloc((size_t)std::max(ntiles, 1))); CUDA_TRY(tilePoseN.alloc((size_t)std::max(ntiles, 1)));
-		if (ntiles > 0) {
-			k_tile_info<<<ntiles, 128, 0, stream>>>(tilePtr.p, tileLm.p, e_ip.p, ntiles, tilePose0.p, tilePoseN.p);
-			launches++;
-			CUDA_TRY(cudaGetLastError());
-			CUDA_TRY(tileInfo.alloc((size_t)ntiles));
-			k_tile_info3<<<ntiles, 128, 0, stream>>>(tilePtr.p, tileLm.p, e_ip.p, e_hpl.p, S.eLocal, S.nhplLocal, ntiles, tileInfo.p);
-			launches++;
-			CUDA_TRY(cudaGetLastError());
-		}
-		CUDA_TRY(cudaFuncSetAttribute(k_linearize_landmark3, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Jh3Smem)));
-		jh3Grid = std::max(1, std::min(ntiles, numSMs * 4));
-		// the tile-local Schur pair is correct but (round 1) slower than k_schur: 387 vs 267 us on kitti00_shaped -> opt-in
-		useSchur2 = cfg.reserved[3] == 2 && S.numP > 0 && S.numL > 0 && ntiles > 0;
-		// 0 / 3 = k_schur3 (destination-sorted products, six lanes per product; default), 5 = landmark tiles on the fp64 tensor pipe
-		// (k_schur_tiles_mma + k_schur_reduce, cuba_schur5.cuh: 12 % faster on the banded 5 M-edge graph, on par on kitti00_shaped,
-		// 2x slower on the real ba_kitti_00 whose loop closures leave 4.4 products per (tile, destination) segment -> opt-in),
-		// 4 = k_schur4 (k_schur3 + cooperative cp.async block loads: slower, kept for the record), 1 = k_schur (lane per product),
-		// 2 = tile-local pair without tensor cores
-		useSchur5 = cfg.reserved[3] == 5 && cfg.reserved[1] != 1 && sizeof(T) == 8 && S.numP > 0 && S.numL > 0 && ntiles > 0 && S.eLocal > 0;
-		useSchur3 = cfg.reserved[3] == 0 || cfg.reserved[3] == 3 || cfg.reserved[3] == 4 || cfg.use_fp32 == 2;
-		if (cfg.use_fp32 == 2) { useSchur2 = false; useSchur5 = false; }
-		if (useSchur3 && S.nmulLocal > 0) {
+		if (S.nmulLocal > 0) {
 			CUDA_TRY(prodL.alloc((size_t)S.nmulLocal));
 			KLAUNCH(schur3::k_prod_landmark, S.nmulLocal, prodI.p, hplLm.p, (int)S.nmulLocal, prodL.p);
 		}
-		if (useSchur5) {
-			// the Schur stage cuts its own, larger landmark tiles (windows of 448 edges)
-			const int tb5 = std::min(S.lmBeg, S.numL), te5 = std::min(S.lmEnd, S.numL) + (S.lmEnd > S.numL ? 1 : 0);
-			s5Ntiles = (S.eLocal + schur5::WINDOW - 1) / schur5::WINDOW;
-			CUDA_TRY(s5TileLm.alloc((size_t)s5Ntiles + 1)); CUDA_TRY(s5TileInfo.alloc((size_t)s5Ntiles));
-			KLAUNCH(sgpu::k_tiles, s5Ntiles + 1, tilePtr.p, tb5, te5, schur5::WINDOW, s5Ntiles, s5TileLm.p);
-			k_tile_info3<<<s5Ntiles, 128, 0, stream>>>(tilePtr.p, s5TileLm.p, e_ip.p, e_hpl.p, S.eLocal, S.nhplLocal, s5Ntiles, s5TileInfo.p);
-			launches++;
-			CUDA_TRY(cudaGetLastError());
-			int rc = setup_schur2(s5TileInfo.p, s5Ntiles); if (rc) return rc;
-			if (useSchur5) {
-				CUDA_TRY(s5SegRec.alloc((size_t)std::max(s2Nseg, 1)));
-				KLAUNCH(schur5::k_seg_records, s2Nseg, s2_segStart.p, s2_segDest.p, s2_segRank.p, s2_segTile.p, blkRow.p, blkCol.p, s5TileInfo.p, s2_p2i.p, s2_p2j.p, s2Nseg, s5SegRec.p);
-				CUDA_TRY(s5Off.alloc((size_t)std::max(s2Nvalid, 1)));
-				KLAUNCH(schur5::k_prod_offsets, s2Nvalid, s2_segStart.p, s2_segTile.p, s5TileInfo.p, s2_p2i.p, s2_p2j.p, s2Nseg, s2Nvalid, s5Off.p);
-				CUDA_TRY(cudaFuncSetAttribute(schur5::k_schur_tiles_mma, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(schur5::Smem)));
-			}
-		}
-		else if (useSchur2) { int rc = setup_schur2(tileInfo.p, ntiles); if (rc) return rc; }
-		tmark("alloc + tile info queued");
+		tmark("alloc queued");
 		if (jhV4) { int rc = setup_jh4(); if (rc) return rc; }
 		tmark("jh4 queued");
 		if (S.numP > 0) { int rc = setup_pcg2(); if (rc) return rc; }        // host-heavy: overlaps the warp-tile kernels queued above
@@ -827,23 +741,13 @@ struct Engine : EngineBase {
 		tmark("pcg partition (host)");
 		if (jhV4) { int rc = setup_jh4_finish(); if (rc) return rc; }
 		tmark("jh4 finish");
-		nChiLin = jhV4 ? jh4Grid : (jhV3 ? jh3Grid : ntiles);
+		nChiLin = jhV4 ? jh4Grid : ntiles;
 		nPoseBlocks = (S.numP + RED_BLOCK - 1) / RED_BLOCK;
 		nChiBlocks = std::max(1, std::min((eL + RED_BLOCK - 1) / RED_BLOCK, numSMs * 8));
 		CUDA_TRY(chiPartial.alloc((size_t)std::max(std::max(ntiles, nChiBlocks), jh4Grid) + 1));
 		CUDA_TRY(scalePartialL.alloc((size_t)std::max(ntiles, (S.numL + RED_BLOCK - 1) / RED_BLOCK) + 1));
 		CUDA_TRY(scalePartialP.alloc((size_t)nPoseBlocks + 1));
 		CUDA_TRY(chiSq.alloc((size_t)S.E));
-		// cooperative grid of the first-generation PCG kernel
-		{
-			int perSM = 0;
-			CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, k_pcg<T>, PCG_BLOCK, 0));
-			if (perSM < 1) return fail(CUBA_ERR_CUDA, "k_pcg cannot be resident");
-			const int wantWarps = std::max(1, S.numP);
-			const int wantBlocks = (wantWarps + PCG_BLOCK / 32 - 1) / (PCG_BLOCK / 32);
-			pcgGrid = std::max(1, std::min(wantBlocks, numSMs * std::min(perSM, 2)));
-			CUDA_TRY(pcgPartial.alloc(2 * (size_t)pcgGrid));
-		}
 		return CUBA_OK;
 	}
 
@@ -915,17 +819,11 @@ struct Engine : EngineBase {
 				int dbg = 0;
 #ifdef CUBA_JH4_DEBUG
 				dbg = getenv("CUBA_JH4_DBG") ? atoi(getenv("CUBA_JH4_DBG")) : 0;
-				if (jh4Nst == 3) { switch (dbg) { case 1: JH4_PICK(4, 3, 1) break; case 2: JH4_PICK(4, 3, 2) break; case 4: JH4_PICK(4, 3, 4) break; case 6: JH4_PICK(4, 3, 6) break;
-					case 7: JH4_PICK(4, 3, 7) break; case 8: JH4_PICK(4, 3, 8) break; case 15: JH4_PICK(4, 3, 15) break; default: dbg = 0; } }
-				else { switch (dbg) { case 8: JH4_PICK(5, 2, 8) break; case 7: JH4_PICK(5, 2, 7) break; default: dbg = 0; } }
+				switch (dbg) { case 1: JH4_PICK(4, 2, 1) break; case 2: JH4_PICK(4, 2, 2) break; case 4: JH4_PICK(4, 2, 4) break; case 6: JH4_PICK(4, 2, 6) break;
+					case 7: JH4_PICK(4, 2, 7) break; case 8: JH4_PICK(4, 2, 8) break; case 15: JH4_PICK(4, 2, 15) break; default: dbg = 0; }
 #endif
 				if (mixed) { fn = (const void*)jh4::k_linearize_landmark4<4, 2, 0, true>; smem = (size_t)2 * jh4::WARPS * sizeof(jh4::StageOf<4, 2>); }
-				if (!fn) {
-					if (jh4Nst == 3) JH4_PICK(4, 3, 0)
-					else if (jh4MinB == 4) JH4_PICK(4, 2, 0)
-					else if (jh4MinB == 5) JH4_PICK(5, 2, 0)
-					else JH4_PICK(6, 2, 0)
-				}
+				if (!fn) JH4_PICK(4, 2, 0)
 				if (fn != jh4AttrSet) { CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); jh4AttrSet = fn; }   // once per kernel, not per launch
 				void* kargs[] = { (void*)&b };
 				CUDA_TRY(cudaLaunchKernel(fn, dim3(jh4Grid), dim3(jh4::WARPS * 32), kargs, smem, stream));
@@ -954,22 +852,7 @@ struct Engine : EngineBase {
 #endif
 			}
 		}
-		else if (jhV3) {
-			if constexpr (sizeof(T) == 8) {
-				LinLm3Args b;
-				b.base = a; b.info = tileInfo; b.ntiles = ntiles;
-				k_linearize_landmark3<<<jh3Grid, JH3_TL, sizeof(Jh3Smem), stream>>>(b);
-			}
-		}
-		else if (jhV2) {
-			LinLm2Args<T> b;
-			b.base = a; b.tilePose0 = tilePose0; b.tilePoseN = tilePoseN; b.eLocal = S.eLocal; b.nhplLocal = S.nhplLocal;
-			k_linearize_landmark2<T><<<ntiles, JH2_TL, 0, stream>>>(b);
-		}
-		else if (tileSize == 128 && jhMinBlocks >= 6) k_linearize_landmark<T, 128, 6><<<ntiles, 128, 0, stream>>>(a);
-		else if (tileSize == 128) k_linearize_landmark<T, 128, 4><<<ntiles, 128, 0, stream>>>(a);
-		else if (jhMinBlocks >= 3) k_linearize_landmark<T, 256, 3><<<ntiles, 256, 0, stream>>>(a);
-		else k_linearize_landmark<T, 256, 2><<<ntiles, 256, 0, stream>>>(a);
+		else k_linearize_landmark<T, LM_TILE, 6><<<ntiles, LM_TILE, 0, stream>>>(a);
 		launches++;
 		CUDA_TRY(cudaGetLastError());
 		return CUBA_OK;
@@ -1075,34 +958,6 @@ struct Engine : EngineBase {
 	int launch_schur(T lambda)
 	{
 		ProfScope ps(this, CUBA_PROF_SCHUR_COMPLEMENT);
-		if (useSchur2 || useSchur5) {
-			schur2::TileArgs<T> ta;
-			ta.Hpl = Hpl; ta.Hll = Hll; ta.bl = bl; ta.info = tileInfo; ta.hplLm = hplLm;
-			ta.tileSegPtr = s2_tileSegPtr; ta.segStart = s2_segStart; ta.segDest = s2_segDest; ta.segRank = s2_segRank; ta.p2i = s2_p2i; ta.p2j = s2_p2j;
-			ta.blkRow = blkRow; ta.blkCol = blkCol; ta.numL = S.numL; ta.lambda = lambda; ta.invHll = invHll; ta.partial = s2_partial;
-			if (useSchur5) {
-				if constexpr (sizeof(T) == 8) {
-					schur5::Args sa;
-					sa.Hpl = Hpl; sa.Hll = Hll; sa.bl = bl; sa.info = s5TileInfo; sa.hplLm = hplLm; sa.tileSegPtr = s2_tileSegPtr; sa.segRec = s5SegRec; sa.off = s5Off;
-					sa.p2i = s2_p2i; sa.p2j = s2_p2j; sa.numL = S.numL; sa.lambda = lambda; sa.invHll = invHll; sa.partial = s2_partial;
-					schur5::k_schur_tiles_mma<<<s5Ntiles, schur5::WARPS * 32, sizeof(schur5::Smem), stream>>>(sa);
-				}
-			}
-			else schur2::k_schur_tiles<T><<<ntiles, schur2::TL, 0, stream>>>(ta);
-			launches++;
-			CUDA_TRY(cudaGetLastError());
-			schur2::ReduceArgs<T> ra;
-			ra.partial = s2_partial; ra.destSegPtr = s2_destSegPtr; ra.Hpp = Hpp; ra.bp = bp;
-			ra.blkRow = blkRow; ra.blkCol = blkCol; ra.u2f = u2f; ra.u2fT = u2fT; ra.nblk = S.nblk; ra.lambda = lambda;
-			ra.addDiag = rank == 0 ? 1 : 0; ra.fVal = fVal; ra.bsc = bsc;
-			schur2::k_schur_reduce<T><<<(S.nblk + 3) / 4, 128, 0, stream>>>(ra);
-			launches++;
-			CUDA_TRY(cudaGetLastError());
-			if (world > 1) {
-				int rc = allreduce(fVal.p, 36 * (size_t)S.nfull + 6 * (size_t)S.numP, true); if (rc) return rc;   // Hsc | bsc: one buffer
-			}
-			return CUBA_OK;
-		}
 		{
 			// the inverses of this rank's landmarks only (nobody reads the others here)
 			const int l0 = std::min(S.lmBeg, S.numL), l1 = std::min(S.lmEnd, S.numL);
@@ -1112,7 +967,7 @@ struct Engine : EngineBase {
 				CUDA_TRY(cudaGetLastError());
 			}
 		}
-		if (useSchur3 && S.numP > 0 && S.numL > 0) {
+		if (S.numP > 0 && S.numL > 0) {
 			schur3::Args<T> a;
 			a.Hpl = Hpl; a.invHll = invHll; a.bl = bl; a.Hpp = Hpp; a.bp = bp;
 			a.prodPtr = prodPtr; a.prodI = prodI; a.prodJ = prodJ; a.prodL = prodL;
@@ -1126,8 +981,7 @@ struct Engine : EngineBase {
 					schur3::k_schur3<double, float><<<(S.nblk + schur3::WARPS - 1) / schur3::WARPS, schur3::WARPS * 32, 0, stream>>>(m);
 				}
 			}
-			else if (cfg.reserved[3] != 4) schur3::k_schur3<T><<<(S.nblk + schur3::WARPS - 1) / schur3::WARPS, schur3::WARPS * 32, 0, stream>>>(a);
-			else schur3::k_schur4<T><<<(S.nblk + schur3::WARPS - 1) / schur3::WARPS, schur3::WARPS * 32, 0, stream>>>(a);
+			else schur3::k_schur3<T><<<(S.nblk + schur3::WARPS - 1) / schur3::WARPS, schur3::WARPS * 32, 0, stream>>>(a);
 			launches++;
 			CUDA_TRY(cudaGetLastError());
 			if (upperReduce) {
@@ -1147,20 +1001,6 @@ struct Engine : EngineBase {
 				}
 			}
 			else if (world > 1) {
-				int rc = allreduce(fVal.p, 36 * (size_t)S.nfull + 6 * (size_t)S.numP, true); if (rc) return rc;   // Hsc | bsc: one buffer
-			}
-		}
-		else if (S.numP > 0 && S.numL > 0) {
-			SchurArgs<T> a;
-			a.Hpl = Hpl; a.invHll = invHll; a.bl = bl; a.Hpp = Hpp; a.bp = bp;
-			a.prodPtr = prodPtr; a.prodI = prodI; a.prodJ = prodJ; a.hplLm = hplLm;
-			a.blkRow = blkRow; a.blkCol = blkCol; a.u2f = u2f; a.u2fT = u2fT; a.nblk = S.nblk;
-			a.lambda = lambda; a.addDiag = rank == 0 ? 1 : 0; a.fVal = fVal; a.bsc = bsc;
-			const int wpb = SCHUR_BLOCK / 32;
-			k_schur<T><<<(S.nblk + wpb - 1) / wpb, SCHUR_BLOCK, 0, stream>>>(a);
-			launches++;
-			CUDA_TRY(cudaGetLastError());
-			if (world > 1) {
 				int rc = allreduce(fVal.p, 36 * (size_t)S.nfull + 6 * (size_t)S.numP, true); if (rc) return rc;   // Hsc | bsc: one buffer
 			}
 		}
@@ -1210,42 +1050,8 @@ struct Engine : EngineBase {
 			CUDA_TRY(w_bigPartial.alloc(std::max<size_t>(big ? 12 * (size_t)ntW : 12, 11 * (size_t)numSMs * 6 * jh4::WARPS)));
 			KLAUNCH(jh4::k_emit, (long long)N * 32, w_start.p, w_pieces.p, w_base.p, N, lmPtr.p, lb, w_levels.p,
 				e_mx.p, e_my.p, e_mz.p, e_om.p, e_ip.p, e_il.p, e_hpl.p, w_tile.p, w_rec.p, w_tilePose.p, w_tilePieces.p);
-			jh4Grid = std::max(1, std::min((ntW + WARPS - 1) / WARPS, numSMs * jh4MinB));
+			jh4Grid = std::max(1, std::min((ntW + WARPS - 1) / WARPS, numSMs * 4));      // 4 CTAs per SM: the shape's __launch_bounds__
 		}
-		return CUBA_OK;
-	}
-
-	// (tile, destination) segments of the block products for the tile-local Schur kernels
-	int setup_schur2(const TileInfo* tinfo, int nt)
-	{
-		using namespace schur2;
-		const int N = (int)S.nmulLocal, nblk = S.nblk;
-		if (N <= 0) { useSchur2 = false; useSchur5 = false; return CUBA_OK; }
-		CUDA_TRY(s2_key.alloc(N)); CUDA_TRY(s2_keyS.alloc(N)); CUDA_TRY(s2_val.alloc(N)); CUDA_TRY(s2_valS.alloc(N));
-		CUDA_TRY(s2_head.alloc(N)); CUDA_TRY(s2_segId.alloc(N)); CUDA_TRY(s2_counts.alloc(1));
-		KLAUNCH(schur2::k_keys, N, prodPtr.p, nblk, prodI.p, N, tinfo, nt, s2_key.p, s2_val.p);
-		int rc = sortPairs(s2_key.p, s2_keyS.p, s2_val.p, s2_valS.p, N, 64); if (rc) return rc;
-		KLAUNCH(schur2::k_heads, N, s2_keyS.p, N, s2_head.p);
-		rc = exclusiveSum(s2_head.p, s2_segId.p, N); if (rc) return rc;
-		schur2::k_counts<<<1, 32, 0, stream>>>(s2_keyS.p, s2_head.p, s2_segId.p, N, s2_counts.p);
-		launches++;
-		schur2::Counts hc;
-		CUDA_TRY(cudaMemcpyAsync(&hc, s2_counts.p, sizeof(hc), cudaMemcpyDeviceToHost, stream));
-		CUDA_TRY(cudaStreamSynchronize(stream));
-		const int nseg = hc.nseg;
-		s2Nseg = nseg; s2Nvalid = hc.nvalid;
-		CUDA_TRY(s2_segStart.alloc((size_t)nseg + 1)); CUDA_TRY(s2_segTile.alloc(nseg)); CUDA_TRY(s2_segDest.alloc(nseg));
-		CUDA_TRY(s2_key3.alloc(nseg)); CUDA_TRY(s2_key3S.alloc(nseg)); CUDA_TRY(s2_val3.alloc(nseg)); CUDA_TRY(s2_val3S.alloc(nseg));
-		CUDA_TRY(s2_segRank.alloc(nseg)); CUDA_TRY(s2_rankDest.alloc(nseg));
-		CUDA_TRY(s2_tileSegPtr.alloc((size_t)nt + 1)); CUDA_TRY(s2_destSegPtr.alloc((size_t)nblk + 1));
-		CUDA_TRY(s2_p2i.alloc(N)); CUDA_TRY(s2_p2j.alloc(N));
-		KLAUNCH(schur2::k_segments, N + 1, s2_keyS.p, s2_valS.p, s2_head.p, s2_segId.p, prodI.p, prodJ.p, N, nseg, hc.nvalid,
-			s2_segStart.p, s2_segTile.p, s2_segDest.p, s2_p2i.p, s2_p2j.p, s2_key3.p, s2_val3.p);
-		KLAUNCH(schur2::k_ptr_from_field, nt + 1, s2_segTile.p, nseg, nt, s2_tileSegPtr.p);
-		rc = sortPairs(s2_key3.p, s2_key3S.p, s2_val3.p, s2_val3S.p, nseg, 32 + sgpu::bits_for((unsigned long long)std::max(nblk, 1))); if (rc) return rc;
-		KLAUNCH(schur2::k_rank, nseg, s2_key3S.p, s2_val3S.p, nseg, s2_segRank.p, s2_rankDest.p);
-		KLAUNCH(schur2::k_ptr_from_field, nblk + 1, s2_rankDest.p, nseg, nblk, s2_destSegPtr.p);
-		CUDA_TRY(s2_partial.alloc((size_t)schur2::PW * std::max(nseg, 1)));
 		return CUBA_OK;
 	}
 
@@ -1448,7 +1254,7 @@ struct Engine : EngineBase {
 	DBuf<unsigned char> p5RowPeers;
 	DBuf<T> p5Linv, p5R0, p5Zhat, p5RcRow, p5Rc0;
 	DBuf<float> p5AcInv;
-	DBuf<double> p5AcP, p5Lp, p5Wp, p5Ld;
+	DBuf<double> p5AcP;
 	DBuf<double> cdM, cdL, cdW, cdDinv;            // dense work matrices of k_coarse_dense
 	bool p5Dense = false;
 	DBuf<unsigned long long> p5Boards;
@@ -1463,7 +1269,6 @@ struct Engine : EngineBase {
 	p5t::Pcg5Dims p5tDims{}, p5tDimsBJ{};            // the tuned one-GPU shape (cuba_pcg5t.cuh), when p5Tuned
 	const void* p5Fn = nullptr;
 	int p5Block = PCG5_BLOCK;
-	int p5Cluster = 0;                             // CTAs of the cluster that factors the coarse matrix (0: one CTA)
 	bool p5CoarseValid = false; int p5CoarseAge = 0; double p5CoarseLambda = 0;
 	size_t p5InvSmem = 0;
 	long long p5TagBound = 0;                      // conservative host-side bound on the device tag base
@@ -1554,7 +1359,7 @@ struct Engine : EngineBase {
 		const int numP = S.numP;
 		if (numP < 1) return CUBA_OK;
 		const int mode = cfg.reserved[0];
-		if (mode == 1 || mode == 2 || mode == 3 || mode == 4) return CUBA_OK;          // an older kernel was asked for explicitly
+		if (mode == 2 || mode == 3 || mode == 4) return CUBA_OK;          // an older kernel was asked for explicitly
 		const bool wantDist = world > 1 && comm && mode != 7 && (mode == 8 || numP >= 2048);
 		const int W = wantDist ? world : 1;
 		int smemMax = 0;
@@ -1637,21 +1442,15 @@ struct Engine : EngineBase {
 		if (getenv("CUBA_PCG_VERBOSE")) fprintf(stderr, "pcg5: world %d G %d gs %d A %d needMax %d maxRows %d blkMax %d maxNeedAgg %d zhInSmem %d sliceRows %d cap %d smem %zu\n",
 			W, G, gs, A, d.needMax, d.maxRows, PP.blkMax, d.maxNeedAgg, d.zhInSmem, d.sliceRows, d.capBlocks, p5Smem);
 		if (getenv("CUBA_PCG_VERBOSE")) fprintf(stderr, "pcg5: shape %s, %d threads\n", p5Big ? "big" : p5Tuned ? "tuned" : "legacy", p5Block);
-		// coarse inverse: packed block triangle in the shared memory of one CTA (A <= 37), of an 8-CTA cluster (A <= 74) or of a
-		// 16-CTA cluster (A <= 148; non-portable cluster size)
-		p5Cluster = A > PCG4_MAXAGG1 ? (A > PCG4_MAXAGG ? 16 : 8) : 0;
+		// coarse inverse: packed block triangle in the shared memory of one CTA (A <= 37), beyond that the dense tile Cholesky on the
+		// whole chip (cuba_coarse_dense.cuh)
+		p5Dense = A > PCG4_MAXAGG1;
 		const size_t nblkPz = (size_t)A * (A + 1) / 2;
-		if (p5Cluster) {
-			const size_t nloc = (nblkPz + p5Cluster - 1) / p5Cluster;
-			p5InvSmem = nloc * 36 * sizeof(double) + 2 * nloc + 16;
-		} else p5InvSmem = (nblkPz + 2 * (size_t)A) * 36 * sizeof(double);
-		if (p5InvSmem + 1024 > (size_t)smemMax) return CUBA_OK;
-		if (p5Cluster == 16) {
-			CUDA_TRY(cudaFuncSetAttribute(k_coarse_chol_cluster2<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p5InvSmem));
-			CUDA_TRY(cudaFuncSetAttribute(k_coarse_chol_cluster2<16>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
-		} else if (p5Cluster == 8) CUDA_TRY(cudaFuncSetAttribute(k_coarse_chol_cluster2<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p5InvSmem));
-		else CUDA_TRY(cudaFuncSetAttribute(k_coarse_invert<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max(p5InvSmem, (!pcg4Cluster && pcg4Ok) ? pcg4InvSmem : 0)));
-		if ((size_t)A * 36 * sizeof(double) > 48 * 1024) CUDA_TRY(cudaFuncSetAttribute(k_coarse_trinv, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)((size_t)A * 36 * sizeof(double))));
+		if (!p5Dense) {
+			p5InvSmem = (nblkPz + 2 * (size_t)A) * 36 * sizeof(double);
+			if (p5InvSmem + 1024 > (size_t)smemMax) return CUBA_OK;
+			CUDA_TRY(cudaFuncSetAttribute(k_coarse_invert<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max(p5InvSmem, (!pcg4Cluster && pcg4Ok) ? pcg4InvSmem : 0)));
+		}
 		CUDA_TRY(p5CtaRow.upload(PP.rows, stream, arena)); CUDA_TRY(p5NeedPtr.upload(PP.nptr, stream, arena)); CUDA_TRY(p5NeedCol.upload(PP.ncol, stream, arena));
 		CUDA_TRY(p5Local.upload(PP.local, stream, arena)); CUDA_TRY(p5RowPeers.upload(peers, stream, arena));
 		CUDA_TRY(p5AggRow.upload(CP.aggRow, stream, arena)); CUDA_TRY(p5NaPtr.upload(CP.naPtr, stream, arena)); CUDA_TRY(p5NaList.upload(CP.naList, stream, arena));
@@ -1661,8 +1460,7 @@ struct Engine : EngineBase {
 		CUDA_TRY(p5Linv.alloc(36 * nP)); CUDA_TRY(p5R0.alloc(6 * nP)); CUDA_TRY(p5Zhat.alloc(36 * nP)); CUDA_TRY(p5RcRow.alloc(6 * nP)); CUDA_TRY(p5Rc0.alloc(std::max(nc, 1)));
 		CUDA_TRY(cZx.alloc(36 * nP)); CUDA_TRY(cU.alloc(36 * (size_t)S.nfull)); CUDA_TRY(cInfo.alloc(1));
 		CUDA_TRY(fHat.alloc(36 * (size_t)S.nfull));
-		CUDA_TRY(p5AcP.alloc(nblkPz * 36)); CUDA_TRY(p5AcInv.alloc((size_t)nc * nc)); CUDA_TRY(p5Lp.alloc(nblkPz * 36)); CUDA_TRY(p5Wp.alloc(nblkPz * 36)); CUDA_TRY(p5Ld.alloc((size_t)A * 36));
-		p5Dense = A > PCG4_MAXAGG1 && !getenv("CUBA_COARSE_CLUSTER");
+		CUDA_TRY(p5AcP.alloc(nblkPz * 36)); CUDA_TRY(p5AcInv.alloc((size_t)nc * nc));
 		if (p5Dense) {
 			const size_t ntd = ((size_t)nc + cdense::NB - 1) / cdense::NB, npd = ntd * cdense::NB;
 			CUDA_TRY(cdM.alloc(npd * npd)); CUDA_TRY(cdL.alloc(npd * npd)); CUDA_TRY(cdW.alloc(npd * npd)); CUDA_TRY(cdDinv.alloc(ntd * cdense::NB * cdense::NB));
@@ -1695,7 +1493,7 @@ struct Engine : EngineBase {
 	}
 
 	// coarse matrix Ac = Z^T S Z of the current system and its inverse (fp32), for the aggregates behind (cbPtr, cbList)
-	int launch_coarse_setup(int A, int cluster, size_t invSmem, const int* cbPtr, const int* cbList, double* AcP, float* AcInv, double* Lp, double* Ld, double* Wp, bool dense = false)
+	int launch_coarse_setup(int A, size_t invSmem, const int* cbPtr, const int* cbList, double* AcP, float* AcInv, bool dense)
 	{
 		const int nblkP = A * (A + 1) / 2;
 		KLAUNCH(k_coarse_project<T>, 36LL * S.nfull, fVal.p, cRowOf.p, fColInd.p, S.nfull, cZx.p, cU.p);
@@ -1710,21 +1508,7 @@ struct Engine : EngineBase {
 			launches++;
 			return CUBA_OK;
 		}
-		if (cluster) {
-			// Cholesky in the shared memory of an 8- or 16-CTA cluster, then the triangular inverse (one CTA per block column) and W^T W on the whole chip
-			cudaLaunchConfig_t lc = {};
-			lc.gridDim = dim3(cluster); lc.blockDim = dim3(1024); lc.dynamicSmemBytes = invSmem; lc.stream = stream;
-			cudaLaunchAttribute at[1];
-			at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = cluster; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-			lc.attrs = at; lc.numAttrs = 1;
-			int* infoP = cInfo.p;
-			if (cluster == 16) CUDA_TRY(cudaLaunchKernelEx(&lc, k_coarse_chol_cluster2<16>, (const double*)AcP, A, Lp, Ld, AcInv, infoP));
-			else CUDA_TRY(cudaLaunchKernelEx(&lc, k_coarse_chol_cluster2<8>, (const double*)AcP, A, Lp, Ld, AcInv, infoP));
-			k_coarse_trinv<<<A, 256, (size_t)A * 36 * sizeof(double), stream>>>(Lp, Ld, A, Wp, cInfo.p);
-			k_coarse_wtw<<<(nblkP * 36 + 255) / 256, 256, 0, stream>>>(Wp, A, AcInv, cInfo.p);
-			launches += 2;
-		}
-		else k_coarse_invert<T><<<1, 1024, invSmem, stream>>>(AcP, A, AcInv, cInfo.p);
+		k_coarse_invert<T><<<1, 1024, invSmem, stream>>>(AcP, A, AcInv, cInfo.p);
 		launches++;
 		CUDA_TRY(cudaGetLastError());
 		return CUBA_OK;
@@ -1756,7 +1540,7 @@ struct Engine : EngineBase {
 			const int refreshEvery = cfg.reserved[4] > 0 ? cfg.reserved[4] : 8;
 			const double lamRatio = (p5CoarseValid && p5CoarseLambda > 0 && curLambda > 0) ? std::max(curLambda / p5CoarseLambda, p5CoarseLambda / curLambda) : 1.0;
 			if (!p5CoarseValid || p5CoarseAge >= refreshEvery || lamRatio > 300.0) {
-				int rc = launch_coarse_setup(A, p5Cluster, p5InvSmem, p5CbPtr, p5CbList, p5AcP, p5AcInv, p5Lp, p5Ld, p5Wp, p5Dense); if (rc) return rc;
+				int rc = launch_coarse_setup(A, p5InvSmem, p5CbPtr, p5CbList, p5AcP, p5AcInv, p5Dense); if (rc) return rc;
 				p5CoarseValid = true; p5CoarseAge = 0; p5CoarseLambda = curLambda;
 			}
 			p5CoarseAge++;
@@ -1822,30 +1606,16 @@ struct Engine : EngineBase {
 		lastPcgTwoLevel = false;
 		// 0 (also 7, 8): automatic = block-Jacobi while a solve converges quickly, two-level afterwards -- k_pcg5 for the two-level solves
 		// (and, when the rows are distributed over the ranks, for every solve), k_pcg3 for the quick block-Jacobi ones on one GPU;
-		// 5: always two-level k_pcg5; 6: always block-Jacobi k_pcg5; 3: always k_pcg4; 4: always k_pcg3; 2: k_pcg2; 1: k_pcg
-		{
-			const int m = cfg.reserved[0];
-			const bool two = tlActive && !forceBlockJacobi;
-			if (p5Ok && (m == 5 || m == 6)) return launch_pcg5(m == 5 && !forceBlockJacobi);
-			if (p5Ok && (m == 0 || m == 7 || m == 8) && (p5Dist || two)) return launch_pcg5(two);
-			if ((m == 0 || m == 7 || m == 8) && !(pcg4Ok && two)) return launch_pcg2(pcg3Ok);
-			if ((m == 0 || m == 7 || m == 8) && pcg4Ok && two) return launch_pcg4();
-		}
-		if (pcg4Ok && cfg.reserved[0] == 3 && !forceBlockJacobi) return launch_pcg4();
-		if (cfg.reserved[0] == 0 || cfg.reserved[0] == 3 || cfg.reserved[0] == 4) return launch_pcg2(pcg3Ok);  // k_pcg3: flag-synchronised exchange (k_pcg2 beyond ~85 rows per CTA)
-		if (cfg.reserved[0] == 2) return launch_pcg2(false);   // k_pcg2: one grid barrier per iteration
-		ProfScope ps(this, CUBA_PROF_DECOMP_NUMERICAL);
-		PcgArgs<T> a;
-		a.fRowPtr = fRowPtr; a.fColInd = fColInd; a.fVal = fVal; a.b = bsc; a.numP = S.numP;
-		a.x = xp; a.r = pr; a.z = pz; a.q = pq; a.p0 = pp0; a.p1 = pp1; a.Minv = Minv; a.partial = pcgPartial;
-		a.maxIters = cfg.pcg_max_iters > 0 ? cfg.pcg_max_iters : std::max(200, 40 * S.numP);
-		const double tol = cfg.pcg_tol > 0 ? cfg.pcg_tol : (sizeof(T) == 8 ? 1e-11 : 1e-6);
-		a.tol2 = tol * tol;
-		a.status = &dScal.p->pcg;
-		void* args[] = { (void*)&a };
-		CUDA_TRY(cudaLaunchCooperativeKernel((void*)k_pcg<T>, dim3(pcgGrid), dim3(PCG_BLOCK), args, 0, stream));
-		launches++;
-		return CUBA_OK;
+		// 5: always two-level k_pcg5; 6: always block-Jacobi k_pcg5; 3: always k_pcg4; 4: always k_pcg3; 2: k_pcg2.
+		// k_pcg3 falls back to k_pcg2 beyond ~85 rows per CTA, k_pcg5 and k_pcg4 to k_pcg3 where their setup declined the system.
+		const int m = cfg.reserved[0];
+		const bool two = tlActive && !forceBlockJacobi;
+		if (p5Ok && (m == 5 || m == 6)) return launch_pcg5(m == 5 && !forceBlockJacobi);
+		if (p5Ok && (m == 0 || m == 7 || m == 8) && (p5Dist || two)) return launch_pcg5(two);
+		if (pcg4Ok && (m == 0 || m == 7 || m == 8) && two) return launch_pcg4();
+		if (pcg4Ok && m == 3 && !forceBlockJacobi) return launch_pcg4();
+		if (m == 2) return launch_pcg2(false);   // k_pcg2: one grid barrier per iteration
+		return launch_pcg2(pcg3Ok);              // k_pcg3: flag-synchronised exchange
 	}
 
 	int launch_backsub(T lambda)
@@ -1860,12 +1630,10 @@ struct Engine : EngineBase {
 					BacksubArgs<double, float> m;
 					m.Hpl = HplF; m.invHll = invHll; m.bl = bl; m.xp = xp; m.ip = e_ip; m.hpl = e_hpl; m.lmPtr = tilePtr; m.tileLm = tileLm;
 					m.numL = S.numL; m.lambda = lambda; m.XwCur = Xw[cur]; m.XwTrial = Xw[cur ^ 1]; m.xl = xl; m.scalePartial = scalePartialL;
-					if (tileSize == 128) k_backsub<double, 128, float><<<ntiles, 128, 0, stream>>>(m);
-					else k_backsub<double, 256, float><<<ntiles, 256, 0, stream>>>(m);
+					k_backsub<double, LM_TILE, float><<<ntiles, LM_TILE, 0, stream>>>(m);
 				}
 			}
-			else if (tileSize == 128) k_backsub<T, 128><<<ntiles, 128, 0, stream>>>(a);
-			else k_backsub<T, 256><<<ntiles, 256, 0, stream>>>(a);
+			else k_backsub<T, LM_TILE><<<ntiles, LM_TILE, 0, stream>>>(a);
 			launches++;
 			CUDA_TRY(cudaGetLastError());
 		}
@@ -2231,6 +1999,11 @@ int cuba_engine_create(const cuba_config* cfg, cuba_engine** out)
 	memset(&c, 0, sizeof(c));
 	c.device = -1; c.deterministic = 1;
 	if (cfg) c = *cfg;
+	// reserved[0..3] select kernels (include/cuba_b200.h): a value that selects none is refused, never run as some other kernel
+	const unsigned accepted[4] = { 0x1fdu /* 0, 2..8 */, 0x3u /* 0, 1 */, 0x11u /* 0, 4 */, 0x9u /* 0, 3 */ };
+	for (int i = 0; i < 4; i++)
+		if (c.reserved[i] < 0 || c.reserved[i] > 31 || !((accepted[i] >> c.reserved[i]) & 1u))
+			return fail(CUBA_ERR_INVALID, "create: cuba_config.reserved[" + std::to_string(i) + "] = " + std::to_string(c.reserved[i]) + " selects no kernel");
 	std::unique_ptr<EngineBase> impl;
 	int rc;
 	if (c.use_fp32 == 1) { auto* e = new Engine<float>(); e->cfg = c; impl.reset(e); rc = e->init(); }

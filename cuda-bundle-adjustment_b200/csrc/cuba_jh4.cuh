@@ -1,9 +1,9 @@
 // cuba_jh4.cuh -- fourth generation of the Jacobian+Hessian landmark pass: WARP tiles.
 //
 // Replaces computeActiveErrorsKernel + constructQuadraticFormKernel (reference src/cuda_block_solver.cu:732-839)
-// for the landmark-side outputs (Hpl, Hll, bl, chi2), like k_linearize_landmark{,2,3} in cuba_kernels.cuh.
+// for the landmark-side outputs (Hpl, Hll, bl, chi2), like k_linearize_landmark in cuba_kernels.cuh.
 //
-// What the ncu source view of k_linearize_landmark3 showed (profiles/r01_ncu_jh3_*): 43 % of the samples sat in
+// What the ncu source view of the third-generation pass (k_linearize_landmark3, since retired) showed (profiles/r01_ncu_jh3_*): 43 % of the samples sat in
 // the per-landmark reduction loop through shared memory (branchy, 35 % of all instructions), 15 % in the
 // cp.async issue code and 15 % at CTA barriers.  This kernel removes all three:
 //   * the unit of work is a WARP tile: whole landmarks packed greedily into <= 32 edge slots (a landmark with
@@ -52,14 +52,11 @@ struct alignas(16) StageT {
 	unsigned long long mbar;
 	unsigned long long pad;
 };
-// variants: (CTAs of 4 warps per SM, pipeline stages) -> landmark window, pose slots.  Shared memory per CTA = 4 * NST stages.
+// (CTAs of 4 warps per SM, pipeline stages) -> landmark window, pose slots.  Shared memory per CTA = 4 * NST stages.
 template <int MINB, int NST> struct Cfg;
 template <> struct Cfg<4, 2> { static constexpr int XW = 32, PC = 32; };   // 7 056 B / stage
-template <> struct Cfg<5, 2> { static constexpr int XW = 24, PC = 23; };   // 5 504 B / stage
-template <> struct Cfg<6, 2> { static constexpr int XW = 16, PC = 19; };   // 4 672 B / stage
-template <> struct Cfg<4, 3> { static constexpr int XW = 16, PC = 19; };   // 4 672 B / stage, prefetch distance 2
 template <int MINB, int NST> using StageOf = StageT<Cfg<MINB, NST>::XW, Cfg<MINB, NST>::PC>;
-static_assert(sizeof(StageOf<6, 2>) - 16 >= CAP * 144 && sizeof(StageOf<5, 2>) - 16 >= CAP * 144, "Hpl staging must fit the stage");
+static_assert(sizeof(StageOf<4, 2>) - 16 >= CAP * 144, "Hpl staging must fit the stage");
 
 struct Args {
 	const double* pose; const double* cam; const double* Xw;

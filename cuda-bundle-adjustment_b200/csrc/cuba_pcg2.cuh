@@ -1,6 +1,6 @@
 // cuba_pcg2.cuh -- persistent, shared-memory-resident block-Jacobi PCG (second generation).
 //
-// Same mathematics as k_pcg (block-Jacobi preconditioned CG on the reduced pose system) but organised
+// Same mathematics as the first-generation k_pcg (since retired; block-Jacobi preconditioned CG on the reduced pose system) but organised
 // for B200 latency instead of generality:
 //   * split preconditioning: with M_i = L_i L_i^T (Cholesky of the 6x6 diagonal blocks) the kernel forms
 //     A^ = L^-1 S L^-T once per solve (diagonal blocks become I) and runs plain CG on A^ y = L^-1 b,

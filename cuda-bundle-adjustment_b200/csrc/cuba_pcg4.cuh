@@ -768,130 +768,8 @@ k_coarse_chol_cluster(const double* __restrict__ AcP, int A, double* Lp, double*
 }
 
 
-// ------------------------------------------------------------------------------------------------------------------
-// Second generation of the cluster Cholesky, for up to 148 aggregates (k_pcg5: one aggregate per CTA, ~9 poses): the packed
-// triangle (148 aggregates: 11 026 blocks, 3.2 MB) needs the shared memory of a 16-CTA cluster (non-portable size, allowed on
-// B200), so everything but the blocks themselves had to leave shared memory: the inverses of the diagonal factors go straight
-// to global memory, the packed-index -> (ib, jb) map is kept only for the CTA's own blocks (2 bytes each).  Same arithmetic
-// and summation order as k_coarse_chol_cluster; CL = 8 or 16 CTAs per cluster, launched with cudaLaunchKernelEx.
-// ------------------------------------------------------------------------------------------------------------------
+// at most one coarse aggregate per CTA of k_pcg5 (about nine poses each)
 constexpr int PCG5_MAXAGG = 148;
-
-template <int CL>
-__global__ void __launch_bounds__(1024, 1) k_coarse_chol_cluster2(const double* __restrict__ AcP, int A, double* Lp, double* Ld, float* AcInv, int* info)
-{
-	namespace cgx = cooperative_groups;
-	cgx::cluster_group cluster = cgx::this_cluster();
-	extern __shared__ __align__(16) unsigned char smem_raw[];
-	const int nblkP = A * (A + 1) / 2, nc = 6 * A;
-	const int nloc = (nblkP + CL - 1) / CL;                        // blocks per CTA
-	double* Bl = reinterpret_cast<double*>(smem_raw);              // [nloc][36] own blocks: local slot lb holds block lb * CL + rank
-	unsigned char* s_ib = reinterpret_cast<unsigned char*>(Bl + (size_t)nloc * 36);   // [nloc] (ib, jb) of the own blocks
-	unsigned char* s_jb = s_ib + nloc;
-	__shared__ int s_fail;
-	__shared__ double s_D[36], s_Li[36], s_id[6];
-	const int rank = (int)cluster.block_rank(), tid = threadIdx.x, NT = blockDim.x;
-	double* base[CL];
-#pragma unroll
-	for (int r = 0; r < CL; r++) base[r] = cluster.map_shared_rank(Bl, r);
-	int* fail0 = cluster.map_shared_rank(&s_fail, 0);
-	auto blk = [&](int ib, int jb) -> double* { const int b = ib * (ib + 1) / 2 + jb; return base[b % CL] + (size_t)(b / CL) * 36; };
-	for (int e = tid; e < nloc * 36; e += NT) {
-		const int b = (e / 36) * CL + rank;
-		Bl[e] = b < nblkP ? AcP[(size_t)b * 36 + (e % 36)] : 0.0;
-	}
-	for (int lb = tid; lb < nloc; lb += NT) {
-		const int b = lb * CL + rank;
-		int ib = (int)((sqrt(8.0 * b + 1.0) - 1.0) * 0.5);
-		while ((ib + 1) * (ib + 2) / 2 <= b) ib++;
-		while (ib * (ib + 1) / 2 > b) ib--;
-		s_ib[lb] = (unsigned char)(b < nblkP ? ib : 255); s_jb[lb] = (unsigned char)(b < nblkP ? b - ib * (ib + 1) / 2 : 255);
-	}
-	if (tid == 0) s_fail = 0;
-	cluster.sync();
-	for (int kb = 0; kb < A; kb++) {
-		if (tid < 32) {
-			// every CTA factors the (already final) diagonal block itself: 6x6 Cholesky (lane r owns row r), then L^-1 column by column
-			double* D = s_D;
-			const double* Dg = blk(kb, kb);
-			for (int e = tid; e < 36; e += 32) D[e] = Dg[e];
-			__syncwarp();
-			const int r = tid;
-			for (int j = 0; j < 6; j++) {
-				const double d = D[j * 6 + j];
-				if (!(d > 0)) { if (r == 0) s_fail = 1; break; }
-				const double sq = sqrt(d);
-				__syncwarp();
-				if (r == j) D[j * 6 + j] = sq;
-				else if (r > j && r < 6) D[j * 6 + r] = D[j * 6 + r] / sq;
-				__syncwarp();
-				if (r > j && r < 6)
-					for (int c = j + 1; c <= r; c++) D[c * 6 + r] -= D[j * 6 + r] * D[j * 6 + c];
-				__syncwarp();
-			}
-			__syncwarp();
-			if (r < 6) {
-				for (int c = r + 1; c < 6; c++) D[c * 6 + r] = 0.0;
-				s_id[r] = 1.0 / D[r * 6 + r];
-			}
-			__syncwarp();
-			if (r < 6) {
-				const int q = r;
-				double col[6];
-				for (int i = 0; i < 6; i++) col[i] = 0.0;
-				col[q] = s_id[q];
-				for (int i = q + 1; i < 6; i++) {
-					double sum = 0;
-					for (int k = q; k < i; k++) sum += D[k * 6 + i] * col[k];
-					col[i] = -sum * s_id[i];
-				}
-				for (int i = 0; i < 6; i++) s_Li[q * 6 + i] = col[i];
-			}
-			__syncwarp();
-			// the factor of the diagonal block and its inverse go straight to the outputs (the shared-memory copy stays raw)
-			if (rank == (((kb * (kb + 1)) / 2 + kb) % CL)) for (int e = tid; e < 36; e += 32) { Lp[((size_t)kb * (kb + 1) / 2 + kb) * 36 + e] = D[e]; Ld[(size_t)kb * 36 + e] = s_Li[e]; }
-		}
-		__syncthreads();
-		if (s_fail) { *fail0 = 1; }                                // every CTA computes the same verdict; rank 0's flag is the shared one
-		if (!s_fail)
-		for (int w = tid; w < nloc * 6; w += NT) {                 // panel: one thread per (own block, row)
-			const int lb = w / 6, r = w - 6 * lb;
-			const int ib = s_ib[lb], jb = s_jb[lb];
-			if (jb != kb || ib <= kb || ib == 255) continue;
-			double* X = Bl + (size_t)lb * 36;
-			double x[6], y[6];
-			for (int k = 0; k < 6; k++) x[k] = X[k * 6 + r];
-			for (int c = 0; c < 6; c++) { double sm = 0; for (int k = 0; k <= c; k++) sm += x[k] * s_Li[k * 6 + c]; y[c] = sm; }
-			for (int c = 0; c < 6; c++) X[c * 6 + r] = y[c];
-		}
-		cluster.sync();
-		if (*fail0) break;
-		for (int w = tid; w < nloc * 36; w += NT) {               // trailing: one thread per (own block, entry)
-			const int lb = w / 36, rc = w - 36 * lb, c = rc / 6, r = rc - 6 * c;
-			const int ib = s_ib[lb], jb = s_jb[lb];
-			if (jb <= kb || ib == 255) continue;                   // ib >= jb > kb
-			const double* P = blk(ib, kb);
-			const double* Q = blk(jb, kb);
-			double sm = 0;
-			for (int k = 0; k < 6; k++) sm += P[k * 6 + r] * Q[k * 6 + c];
-			Bl[(size_t)lb * 36 + rc] -= sm;
-		}
-		cluster.sync();
-	}
-	if (*fail0) {
-		for (int e = rank * NT + tid; e < nc * nc; e += CL * NT) AcInv[e] = 0.f;
-		if (rank == 0 && tid == 0 && info) *info = 1;
-		cluster.sync();
-		return;
-	}
-	// the off-diagonal blocks of the factor L (packed, block b at Lp + 36 b) leave for k_coarse_trinv
-	for (int e = tid; e < nloc * 36; e += NT) {
-		const int lb = e / 36, b = lb * CL + rank;
-		if (b < nblkP && s_ib[lb] != s_jb[lb]) Lp[(size_t)b * 36 + (e % 36)] = Bl[e];
-	}
-	if (rank == 0 && tid == 0 && info) *info = 0;
-	cluster.sync();                                            // nobody leaves while its shared memory may still be read
-}
 
 // W = L^-1 (block lower triangular), one CTA per block column jb: W(jb,jb) = L_jj^-1,
 // W(ib,jb) = -L_ii^-1 sum_{k=jb}^{ib-1} L(ib,k) W(k,jb).  The columns are independent; a column is sequential in ib.

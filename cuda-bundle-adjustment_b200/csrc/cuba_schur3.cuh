@@ -1,4 +1,4 @@
-// cuba_schur3.cuh -- Schur complement, third kernel: one warp per destination block like k_schur (products
+// cuba_schur3.cuh -- Schur complement, third kernel: one warp per destination block like the first kernel, k_schur (since retired; products
 // sorted by destination at structure time -> every block is a fixed-order sum, no fp64 atomics; reference
 // src/cuda_block_solver.cu:955-977 does 36 atomics per product), but SIX lanes per product instead of one.
 //
@@ -124,148 +124,6 @@ __global__ void k_expand_upper(const T* __restrict__ uVal, const int* __restrict
 	const T v = uVal[w];
 	fVal[36 * (size_t)u2f[k] + e] = v;
 	if (blkRow[k] != blkCol[k]) fVal[36 * (size_t)u2fT[k] + r * 6 + c] = v;
-}
-
-}  // namespace schur3
-}  // namespace cuba_b200
-
-// ------------------------------------------------------------------------------------------------------------
-// k_schur4 (experiment, cfg.reserved[3] == 4): k_schur3 with warp-cooperative block loads.  Hypothesis: the gather
-// kernels are bound by the L1TEX tag stage (every load instruction of k_schur3 touches five different blocks).
-// MEASURED SLOWER (kitti00_shaped: 355 us vs 278 us for k_schur3, 310 us for k_schur) -- the hypothesis was wrong or the
-// extra shared-memory round trip costs more than it saves; kept because the parity test pins it to k_schur3's bits.
-// The ten 144-byte Hpl blocks and the five 72-byte inverses of a step are fetched with
-// 16-byte / 8-byte cp.async copies laid out so that consecutive lanes cover consecutive bytes of a block
-// (~40 look-ups per step), double buffered in shared memory per warp, and the arithmetic reads them back as
-// shared-memory broadcasts.  Same fixed summation order as k_schur3.
-// ------------------------------------------------------------------------------------------------------------
-namespace cuba_b200 {
-namespace schur3 {
-
-template <typename T>
-struct alignas(16) WarpBuf {
-	T blk[2][2 * SLOTS][18];      // [stage][0..4: Hpl_i of the slot, 5..9: Hpl_j][18]
-	T inv[2][SLOTS][10];          // [stage][slot][9 entries of invHll + pad]
-};
-
-template <typename T> __device__ __forceinline__ void cp_chunk(T* smem, const T* g);
-template <> __device__ __forceinline__ void cp_chunk<double>(double* smem, const double* g) { cp_async16(smem, g); }     // 2 doubles
-template <> __device__ __forceinline__ void cp_chunk<float>(float* smem, const float* g) { cp_async8(smem, g); }          // 2 floats
-template <typename T> __device__ __forceinline__ void cp_one(T* smem, const T* g);
-template <> __device__ __forceinline__ void cp_one<double>(double* smem, const double* g) { cp_async8(smem, g); }
-template <> __device__ __forceinline__ void cp_one<float>(float* smem, const float* g) { cp_async4(smem, g); }
-
-template <typename T>
-__global__ void __launch_bounds__(WARPS * 32, 3) k_schur4(const Args<T> a)
-{
-	__shared__ WarpBuf<T> s_buf[WARPS];
-	const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-	const int k = blockIdx.x * WARPS + wid;
-	if (k >= a.nblk) return;
-	WarpBuf<T>& wb = s_buf[wid];
-	const int ra = a.blkRow[k], cb = a.blkCol[k];
-	const bool diag = ra == cb;
-	const int n0 = a.prodPtr[k], n1 = a.prodPtr[k + 1];
-	const int nsteps = (n1 - n0 + SLOTS - 1) / SLOTS;
-	const int slot = lane / 6, r = lane - 6 * slot;
-	const bool worker = slot < SLOTS;
-
-	// loader role of this lane: three 2-scalar chunks of the ten blocks, up to two scalars of the five inverses
-	int lb[3], lp[3];              // block (0..9) and piece (0..8) of chunk lane + 32 q
-#pragma unroll
-	for (int q = 0; q < 3; q++) { const int c = lane + 32 * q; lb[q] = c < 90 ? c / 9 : -1; lp[q] = c % 9; }
-	const int is0 = lane / 9, ip0 = lane - 9 * is0;                   // scalar lane of the inverses (45 scalars: lane, lane + 32)
-	const int is1 = (lane + 32) / 9, ip1 = (lane + 32) - 9 * is1;     // valid when lane + 32 < 45
-
-	auto load_idx = [&](int s, int (&ix)[6]) {
-		// ix[0..2]: Hpl block of the lane's three chunks, ix[3..4]: landmark of its inverse scalars, ix[5]: prodI of its compute slot
-		const int base = n0 + SLOTS * s;
-#pragma unroll
-		for (int q = 0; q < 3; q++) {
-			ix[q] = -1;
-			if (lb[q] >= 0) {
-				const int sl = lb[q] >= SLOTS ? lb[q] - SLOTS : lb[q];
-				const int n = base + sl;
-				if (n < n1) {
-					const int pi = a.prodI[n];
-					ix[q] = (lb[q] >= SLOTS && pi >= 0) ? a.prodJ[n] : pi;
-				}
-			}
-		}
-		ix[3] = (base + is0 < n1) ? a.prodL[base + is0] : -1;
-		ix[4] = (lane + 32 < 45 && base + is1 < n1) ? a.prodL[base + is1] : -1;
-		ix[5] = (worker && base + slot < n1) ? a.prodI[base + slot] : -1;
-	};
-	auto issue = [&](int st, const int (&ix)[6]) {
-#pragma unroll
-		for (int q = 0; q < 3; q++)
-			if (ix[q] >= 0) cp_chunk<T>(&wb.blk[st][lb[q]][2 * lp[q]], a.Hpl + 18 * (size_t)ix[q] + 2 * lp[q]);
-		if (ix[3] >= 0) cp_one<T>(&wb.inv[st][is0][ip0], a.invHll + 9 * (size_t)ix[3] + ip0);
-		if (ix[4] >= 0) cp_one<T>(&wb.inv[st][is1][ip1], a.invHll + 9 * (size_t)ix[4] + ip1);
-		asm volatile("cp.async.commit_group;" ::: "memory");
-	};
-
-	T C[6], vr = T(0);
-#pragma unroll
-	for (int c = 0; c < 6; c++) C[c] = T(0);
-	int ixA[6], ixB[6];
-	load_idx(0, ixA);
-	issue(0, ixA);
-	int have = ixA[5];
-	if (nsteps > 1) load_idx(1, ixA);
-	for (int s = 0; s < nsteps; s++) {
-		const int st = s & 1;
-		int haveNext = -1;
-		if (s + 1 < nsteps) { __syncwarp(); issue(st ^ 1, ixA); haveNext = ixA[5]; }
-		else asm volatile("cp.async.commit_group;" ::: "memory");
-		if (s + 2 < nsteps) load_idx(s + 2, ixB);
-		asm volatile("cp.async.wait_group 1;" ::: "memory");
-		__syncwarp();
-		if (have >= 0) {
-			const T* Ai = wb.blk[st][slot];
-			const T* Aj = wb.blk[st][SLOTS + slot];
-			const T* iv = wb.inv[st][slot];
-			const T a0 = Ai[r], a1 = Ai[6 + r], a2 = Ai[12 + r];
-			const T i0 = iv[0], i1 = iv[3], i2 = iv[6], i3 = iv[4], i4 = iv[7], i5 = iv[8];
-			const T w0 = a0 * i0 + a1 * i1 + a2 * i2;
-			const T w1 = a0 * i1 + a1 * i3 + a2 * i4;
-			const T w2 = a0 * i2 + a1 * i4 + a2 * i5;
-#pragma unroll
-			for (int c = 0; c < 6; c++) C[c] += w0 * Aj[c] + w1 * Aj[6 + c] + w2 * Aj[12 + c];
-			if (diag) {
-				const int cl = a.prodL[n0 + SLOTS * s + slot];
-				const T* b3 = a.bl + 3 * (size_t)cl;
-				vr += w0 * __ldg(b3) + w1 * __ldg(b3 + 1) + w2 * __ldg(b3 + 2);
-			}
-		}
-		have = haveNext;
-#pragma unroll
-		for (int q = 0; q < 6; q++) ixA[q] = ixB[q];
-	}
-	asm volatile("cp.async.wait_group 0;" ::: "memory");
-	__syncwarp();
-	// fixed-order sum over the five slots (the block buffer is free now)
-	T* red = &wb.blk[0][0][0];      // [slot][row][8]: 5*6*8 = 240 <= 2*10*18
-	if (worker) {
-#pragma unroll
-		for (int c = 0; c < 6; c++) red[(slot * 6 + r) * 8 + c] = C[c];
-		red[(slot * 6 + r) * 8 + 6] = vr;
-	}
-	__syncwarp();
-	for (int e = lane; e < 42; e += 32) {
-		const int c = e < 36 ? e / 6 : 6, rr = e < 36 ? e - 6 * c : e - 36;
-		T s = T(0);
-#pragma unroll
-		for (int q = 0; q < SLOTS; q++) s += red[(q * 6 + rr) * 8 + c];
-		if (e < 36) {
-			T val = -s;
-			if (diag && a.addDiag) val += a.Hpp[36 * (size_t)ra + e] + (rr == c ? a.lambda : T(0));
-			a.fVal[36 * (size_t)a.u2f[k] + e] = val;
-			if (!diag) a.fVal[36 * (size_t)a.u2fT[k] + rr * 6 + c] = val;
-		} else if (diag) {
-			a.bsc[6 * (size_t)ra + rr] = (a.addDiag ? a.bp[6 * (size_t)ra + rr] : T(0)) - s;
-		}
-	}
 }
 
 }  // namespace schur3

@@ -82,14 +82,13 @@ typedef struct cuba_config {
 	                          >= 2048 free poses k_pcg5 runs with the block rows DISTRIBUTED over the ranks (NVLink peer boards);
 	                          7 = never distribute (replicated solve), 8 = always distribute.  5 = always two-level k_pcg5,
 	                          6 = always block-Jacobi k_pcg5, 3 = always k_pcg4 (two-level, one grid barrier per iteration),
-	                          4 = always k_pcg3, 2 = k_pcg2 (one grid barrier per iteration), 1 = k_pcg (first generation)
+	                          4 = always k_pcg3, 2 = k_pcg2 (one grid barrier per iteration)
 	                          reserved[1]: 1 = build the index structures on the host (cuba_structure.cpp) instead of
 	                          on the device (cuba_structure_gpu.cuh, default); both give identical structures
-	                          reserved[2]: J+H landmark kernel, 0 = k_linearize_landmark4 (warp tiles, default; 8/9 = 5/6 CTAs per SM,
-	                          7 = three pipeline stages), 6 = k_linearize_landmark3, 5 = ..._landmark2, 1-4 = first generation
-	                          reserved[3]: Schur kernel, 0 = k_schur3 (six lanes per product, default), 1 = k_schur (lane per product),
-	                          2 = tile-local pair (cuba_schur2.cuh), 4 = k_schur4 (cooperative loads; slower), 5 = landmark tiles on the
-	                          fp64 tensor pipe (cuba_schur5.cuh, DMMA m8n8k4; wins only on banded graphs)
+	                          reserved[2]: J+H landmark kernel, 0 = k_linearize_landmark4 (warp tiles, default; fp32: first generation),
+	                          4 = first generation (k_linearize_landmark, 128-edge tiles)
+	                          reserved[3]: Schur kernel, 0 or 3 = k_schur3 (six lanes per product)
+	                          Any other value of reserved[0..3] makes cuba_engine_create fail with CUBA_ERR_INVALID.
 	                          reserved[4]: two-level PCG: solves between rebuilds of the coarse matrix (<=0: 8)
 	                          reserved[5]: automatic solver: block-Jacobi iteration count that switches to two-level (<=0: 100)
 	                          reserved[6]: two-level PCG: upper bound on the number of pose aggregates (<=0: 74; <= 37 uses the one-CTA inverse) */

@@ -252,11 +252,10 @@ def test_two_gpu_trajectory_matches_oracle():
         assert r["chi2_rel_diff_vs_oracle"] < TOL and r["state_diff"] < 1e-9 and r["repeat_diff"] == 0.0, r
 
 
-@pytest.mark.parametrize("variant", [0, 5, 6, 3, 4, 2, 1])
+@pytest.mark.parametrize("variant", [0, 5, 6, 3, 4, 2])
 def test_all_pcg_kernels_solve_the_same_system(pkg, oracle, problems, variant):
     """automatic policy (0), k_pcg5 two-level (5) and block-Jacobi (6) (flag-synchronised, the kernel that also runs distributed
-    over the ranks), two-level k_pcg4 (3), k_pcg3 (4, flag-synchronised), k_pcg2 (single barrier) and k_pcg (first generation)
-    against the direct solve"""
+    over the ranks), two-level k_pcg4 (3), k_pcg3 (4, flag-synchronised) and k_pcg2 (single barrier) against the direct solve"""
     prob = problems("kitti07_shaped"); rk = KERNELS["huber"]
     eng = make_engine(pkg, prob, rk, pcg_variant=variant)
     o = oracle.Oracle(prob, *rk)
@@ -345,27 +344,19 @@ def test_device_and_host_structure_builders_agree(pkg, problems, name):
 
 
 @pytest.mark.parametrize("name", ["small", "kitti07_shaped", "ba_kitti_00", "kitti00_sub"])
-def test_schur_kernels_agree(pkg, oracle, problems, name):
-    """k_schur3 (six lanes per product, default) vs landmark tiles on the fp64 tensor pipe (cuba_schur5.cuh, DMMA) vs k_schur4
-    (+ cooperative loads, same bits as k_schur3) vs k_schur (lane per product) vs the tile-local pair without tensor cores
-    (cuba_schur2.cuh) vs the oracle"""
+def test_schur3_matches_oracle(pkg, oracle, problems, name):
+    """k_schur3 (six lanes per product) against the oracle, on the real-data pieces too"""
     if name.startswith("ba_") and not have_fixture(name):
         pytest.skip("reference fixture absent")
     prob = problems(name); rk = KERNELS["huber"]
-    a = make_engine(pkg, prob, rk, schur_variant=2); b = make_engine(pkg, prob, rk, schur_variant=3); c = make_engine(pkg, prob, rk, schur_variant=1)
-    d = make_engine(pkg, prob, rk, schur_variant=4); e = make_engine(pkg, prob, rk, schur_variant=5)
+    b = make_engine(pkg, prob, rk)
     o = oracle.Oracle(prob, *rk)
-    a.linearize(); b.linearize(); c.linearize(); d.linearize(); e.linearize(); o.compute_errors(); o.build_system()
+    b.linearize(); o.compute_errors(); o.build_system()
     for lam in (1e3, 1.0):
-        assert a.solve(lam)[1] and b.solve(lam)[1] and c.solve(lam)[1] and d.solve(lam)[1] and e.solve(lam)[1] and o.solve(lam)
-        for x, y in zip(d.schur(), b.schur()):
-            assert np.array_equal(x, y)        # k_schur3 and k_schur4 sum in the same order
-        for nme, x, y, w, v, z in zip(("Hsc", "bsc", "invHll"), a.schur(), b.schur(), c.schur(), e.schur(), o.schur()):
-            assert relerr(x, y) < 1e-12, nme
-            assert relerr(w, y) < 1e-12, nme
-            assert relerr(v, y) < 1e-12, nme
-            assert relerr(v, z) < STAGE_TOL, nme
-    a.close(); b.close(); c.close(); d.close(); e.close()
+        assert b.solve(lam)[1] and o.solve(lam)
+        for nme, y, z in zip(("Hsc", "bsc", "invHll"), b.schur(), o.schur()):
+            assert relerr(y, z) < STAGE_TOL, nme
+    b.close()
 
 
 def test_rejects_bad_problems(pkg, problems):
@@ -504,15 +495,15 @@ def test_full_size_properties(pkg, problems):
 
 
 @pytest.mark.parametrize("name", ["small", "kitti07_shaped", "ba_kitti_00", "kitti00_sub"])
-def test_jh_landmark_kernels_agree(pkg, oracle, problems, name):
-    """k_linearize_landmark4 (warp tiles, default) vs generations 3, 2 and 1 of the J+H landmark pass: same Hpl/Hll/bl/chi2
-    to rounding (the kernels group the per-landmark sums differently).  The real ba_kitti_00 has 203 landmarks with
+def test_jh_landmark4_agrees_with_first_generation(pkg, oracle, problems, name):
+    """k_linearize_landmark4 (warp tiles, default) vs the first-generation J+H landmark pass (the fp32 engine's): same
+    Hpl/Hll/bl/chi2 to rounding (the kernels group the per-landmark sums differently).  The real ba_kitti_00 has 203 landmarks with
     more than 32 observations, which the warp-tile kernel cuts into pieces (k_big_reduce); kitti00_sub keeps 8 of them."""
     if name.startswith("ba_") and not have_fixture(name):
         pytest.skip("reference fixture absent")
     prob = problems(name); rk = KERNELS["huber"]
     ref = None
-    for v in (0, 6, 5, 4):
+    for v in (0, 4):
         eng = make_engine(pkg, prob, rk, jh_variant=v)
         chi = eng.linearize()
         out = (np.array([chi]),) + tuple(eng.system())

@@ -1,5 +1,5 @@
 """J+H landmark-pass variants: device time per launch (L2 flushed) on one workload.
-usage: python tools/jh_variants.py [--variants 0,6,5,4] <workload | ba_kitti_00 | ba_kitti_07> ..."""
+usage: python tools/jh_variants.py [--variants 0,4] <workload | ba_kitti_00 | ba_kitti_07> ..."""
 import os
 import sys
 
@@ -9,7 +9,7 @@ import __graft_entry__ as ge  # noqa: E402
 
 pkg = ge.load_package()
 args = sys.argv[1:]
-variants = (0, 8, 7, 6)
+variants = (0, 4)
 if args and args[0] == "--variants":
     variants = tuple(int(v) for v in args[1].split(","))
     args = args[2:]

@@ -1,5 +1,5 @@
-"""Per-stage device times (L2 flushed) for one or more workloads and Schur variants.
-usage: python tools/stage_bench.py [--schur 0,1] <workload | ba_kitti_00> ..."""
+"""Per-stage device times (L2 flushed) for one or more workloads.
+usage: python tools/stage_bench.py <workload | ba_kitti_00> ..."""
 import os
 import sys
 
@@ -9,10 +9,6 @@ import __graft_entry__ as ge  # noqa: E402
 
 pkg = ge.load_package()
 args = sys.argv[1:]
-schur = (0,)
-if args and args[0] == "--schur":
-    schur = tuple(int(v) for v in args[1].split(","))
-    args = args[2:]
 NAMES = {1: "jh_landmark", 2: "jh_pose", 3: "schur", 4: "pcg", 5: "backsub+update+chi2", 6: "chi2"}
 for workload in args or ["kitti00_shaped"]:
     if workload.startswith("ba_"):
@@ -23,17 +19,16 @@ for workload in args or ["kitti00_shaped"]:
     else:
         g = pkg.synth.make_config(workload)
     prob = pkg.graphio.flatten(g)
-    for sv in schur:
-        eng = pkg.Engine(device=0, schur_variant=sv, use_fp32=("mixed" if os.environ.get("MIXED") else False))
-        if os.environ.get("CUBA_DRY_SHARD"):
-            r, w = os.environ["CUBA_DRY_SHARD"].split("/")
-            eng.set_comm(int(r), int(w), b"\0" * 128)
-        eng.initialize(prob)
-        eng.linearize()
-        lam = 1e-5 * eng.max_diagonal()
-        eng.solve(lam)
-        out = []
-        for st in (1, 2, 3, 5, 6):
-            out.append("%s %.1f us" % (NAMES[st], 1e3 * eng.bench_stage(st, reps=20, flush_l2=True, lam=lam)))
-        print("%s schur_variant %d: %s" % (workload, sv, "; ".join(out)), flush=True)
-        eng.close()
+    eng = pkg.Engine(device=0, use_fp32=("mixed" if os.environ.get("MIXED") else False))
+    if os.environ.get("CUBA_DRY_SHARD"):
+        r, w = os.environ["CUBA_DRY_SHARD"].split("/")
+        eng.set_comm(int(r), int(w), b"\0" * 128)
+    eng.initialize(prob)
+    eng.linearize()
+    lam = 1e-5 * eng.max_diagonal()
+    eng.solve(lam)
+    out = []
+    for st in (1, 2, 3, 5, 6):
+        out.append("%s %.1f us" % (NAMES[st], 1e3 * eng.bench_stage(st, reps=20, flush_l2=True, lam=lam)))
+    print("%s: %s" % (workload, "; ".join(out)), flush=True)
+    eng.close()
